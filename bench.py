@@ -29,12 +29,16 @@ One JSON line is printed by rank 0.  Extra objects: `roofline` (dominant kernel,
 `other_configs` (BASELINE configs[1], [3], [4] with their own roofline and parity sample), `clocks`.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
 import sys
 import tempfile
 import time
+
+# the tree bench.py runs from may be read-only: import the project without writing __pycache__ into it
+sys.dont_write_bytecode = True
 
 # the reference arm must see all host cores: torchrun exports OMP_NUM_THREADS=1, and OpenBLAS / libgomp read the
 # environment when they are loaded, i.e. before anything below imports numpy / scipy
@@ -52,6 +56,7 @@ WORKLOAD = dict(V=50000, T=200, E=32, eps=8)
 METRIC = "voxel-pair correlations/sec"
 UNIT = "corr/s"
 SEED = 1234567890
+DUMP_BYTES = 48 << 20       # --dump-outputs: at most this many bytes of kernels
 
 
 def workload_string(V, T, E, eps):
@@ -72,7 +77,23 @@ def parse():
     ap.add_argument("--no-others", action="store_true", help="skip the other BASELINE configs")
     ap.add_argument("--no-ipc", action="store_true", help="epoch exchange through NCCL all-gather instead of CUDA IPC copies")
     ap.add_argument("--clock-interval-ms", type=int, default=20, help="nvidia-smi sampling interval")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the [V, E, E] kernels of the last one to DIR/kernels.npy (float32); "
+                         "when they exceed %d MB, the rows of a fixed sample (dump_rows: seeded, sorted)" % (DUMP_BYTES >> 20))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the kernels of the b200 arm")
+    return args
+
+
+def dump_rows(V, E):
+    """Rows of the kernels --dump-outputs writes: all of them, or a sample fixed by SEED that fits DUMP_BYTES."""
+    n = min(V, DUMP_BYTES // (E * E * 4))
+    if n == V:
+        return np.arange(V)
+    return np.sort(np.random.RandomState(SEED).choice(V, n, replace=False))
 
 
 def make_epoch(e, T, V, out=None):
@@ -266,10 +287,9 @@ def run_reference_arm(args):
     fn, kind, cores = reference_task_fn(host, eps)
     rows = 64                                     # the reference's default voxel_unit
     # a "step" of this arm = one task of 64 voxel rows (bounded sample of the same workload); the value is taken from
-    # the MEDIAN task time of max(steps, 20) tasks after `warmup` tasks, extrapolated by the metric (linear in the
+    # the MEDIAN task time of `steps` tasks after `warmup` tasks, extrapolated by the metric (linear in the
     # number of tasks: every task contracts 64 rows with all V columns of all E epochs)
-    ntasks = max(args.steps, 20)
-    med, done, times = time_reference_tasks(fn, V, ntasks, 120.0, rows=rows, warm=max(args.warmup, 1))
+    med, done, times = time_reference_tasks(fn, V, args.steps, float("inf"), rows=rows, warm=max(args.warmup, 1))
     value = rows * float(V) * E / med
     sample = ("median of %d tasks of %d voxel rows x V=%d x E=%d (kernel path a4+a6+a7 = voxelselector.py:492-505, no CV), "
               "%d BLAS/OpenMP threads" % (done, rows, V, E, cores))
@@ -357,6 +377,7 @@ def run_b200_arm(args):
     lib = _lib.load()
     _lib.require_device()
     sampler = ClockSampler(local, args.clock_interval_ms)
+    atexit.register(sampler.close)      # no nvidia-smi left running, whatever ends the run
     if rank == 0:
         sampler.start()
     peaks = {}
@@ -521,6 +542,22 @@ def run_b200_arm(args):
     ms_step = ms_total / args.steps
     corr_total = float(V) * V * E
     value = corr_total / (ms_step * 1e-3)
+
+    # the kernels of the last timed step, before anything below computes into the same buffers
+    if args.dump_outputs:
+        idx = torch.from_numpy(dump_rows(V, E)).to(dev)
+        if world == 1:
+            sel = Kfull[idx]
+        else:
+            lo = rank * per                 # Kmine holds rows [lo, lo + per); the other ranks add zeros
+            mine = (idx >= lo) & (idx < lo + per)
+            sel = torch.zeros((len(idx), E, E), dtype=torch.float32, device=dev)
+            sel[mine] = Kmine[idx[mine] - lo]
+            dist.reduce(sel, dst=0)
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "kernels.npy"), sel.cpu().numpy())
+        del sel
 
     # per-rank time of the shard alone (no collective): the load balance of the equal-area partition
     balance = None

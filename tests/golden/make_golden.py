@@ -115,7 +115,10 @@ def gen_vs_mid(m):
         raw=np.stack(raw), labels=np.array(labels), eps=eps, task=np.array(task),
         corr_raw=r, corr_norm=z, kernels=k,
         d1=np.stack(d1), d2=np.stack(d2), labels2=np.array(labels2), task2=np.array(task2),
-        corr_raw2=r2, corr_norm2=z2, kernels2=k2,
+        corr_raw2=r2, corr_norm2=z2, kernels2=k2)
+    # the full run in a file of its own: each fixture stays under 1 MB
+    np.savez_compressed(
+        os.path.join(OUT, "vs_mid_run.npz"),
         rawf=np.stack(rawf), labelsf=np.array(labelsf), epsf=epsf, accf=accf, kernelsf=kf)
     print("vs_mid: top voxels", np.argsort(-accf, kind="stable")[:12], "acc", np.sort(accf)[-12:])
 
@@ -265,11 +268,70 @@ def gen_vs_sym(m):
     print("vs_sym: top voxels", np.argsort(-acc, kind="stable")[:10], "acc", np.sort(acc)[-10:])
 
 
+def ref_rows(m, raw, labels, eps, folds, s0, n0, mask_self=False):
+    """Rows [s0, s0+n0) through the reference's stages (voxelselector.py:492-509): shrunk kernels and cross-validation
+    accuracies.  mask_self: zero the self column after its normaliser."""
+    vs = m.VoxelSelector(labels, eps, folds, raw, voxel_unit=n0, process_num=0)
+    clf = svm.SVC(kernel="precomputed", shrinking=False, C=1)
+    corr = vs._correlation_computation((s0, n0))
+    m.fcma_extension.normalization(corr, eps)
+    if mask_self:
+        for i in range(n0):
+            corr[i, :, s0 + i] = 0
+    K = vs._prepare_for_cross_validation(corr, clf)
+    acc = np.array([a for _, a in vs._do_cross_validation(clf, K, (s0, n0))])
+    return K, acc
+
+
+def input_probe(raw, seed, n=64):
+    """n seeded input values (epoch, TR, voxel): the tests regenerate these large inputs and check them against this."""
+    rng = RandomState(seed)
+    idx = np.stack([rng.randint(0, len(raw), n), rng.randint(0, raw[0].shape[0], n),
+                    rng.randint(0, raw[0].shape[1], n)], axis=1)
+    return idx, np.array([raw[e][t, v] for e, t, v in idx], np.float32)
+
+
+def gen_vs_scale(m):
+    """Sampled rows of the BASELINE config shapes (inputs too large to store: regenerated by the tests from
+    synthetic.make_epochs and checked against a probe) and the result-level noise floor case."""
+    out = {}
+    # configs[1]: V = 30 000, T = 200, E = 16, eps = 8, 2 folds; first pass, a middle pass, the ragged tail
+    V, T, E, eps = 30000, 200, 16, 8
+    raw, labels = synthetic.make_epochs(V, T, E)
+    out["c1_probe_idx"], out["c1_probe"] = input_probe(raw, 1)
+    out["c1_rows"] = np.array([64, 15008, V - 32])
+    ks, accs_ = zip(*[ref_rows(m, raw, labels, eps, 2, s0, 32) for s0 in out["c1_rows"]])
+    out["c1_kernels"], out["c1_acc"] = np.stack(ks), np.stack(accs_)
+    # configs[4] shape class: V = 20 000, T = 200, E = 32, eps = 8; kernels only (symmetric: upper triangle stored)
+    V, T, E, eps = 20000, 200, 32, 8
+    raw, labels = synthetic.make_epochs(V, T, E)
+    out["c4_probe_idx"], out["c4_probe"] = input_probe(raw, 4)
+    out["c4_rows"] = np.array([256, 10016, V - 32])
+    ks = np.stack([ref_rows(m, raw, labels, eps, 4, s0, 32)[0] for s0 in out["c4_rows"]])
+    assert np.array_equal(ks, ks.transpose(0, 1, 3, 2))
+    iu = np.triu_indices(E)
+    out["c4_kernels_triu"] = ks[:, :, iu[0], iu[1]]
+    # noise floor: V = 768, T = 200, E = 32, eps = 8, 4 folds; every voxel, on the inputs, on TR-permuted inputs and with
+    # the self column masked
+    V, T, E, eps = 768, 200, 32, 8
+    raw, labels = synthetic.make_epochs(V, T, E)
+    out["nf_probe_idx"], out["nf_probe"] = input_probe(raw, 768)
+    perm = RandomState(7).permutation(T)
+    raw_p = [np.ascontiguousarray(x[perm]) for x in raw]
+    out["nf_acc"] = ref_rows(m, raw, labels, eps, 4, 0, V)[1]
+    out["nf_acc_perm"] = ref_rows(m, raw_p, labels, eps, 4, 0, V)[1]
+    out["nf_acc_masked"] = ref_rows(m, raw, labels, eps, 4, 0, V, mask_self=True)[1]
+    np.savez_compressed(os.path.join(OUT, "vs_scale.npz"), **out)
+    print("vs_scale: noise floor %.3f" % np.mean(out["nf_acc"] != out["nf_acc_perm"]))
+
+
 def main():
     m = reference.load()
-    if len(sys.argv) > 1 and sys.argv[1] == "vs_sym":      # add this fixture without regenerating the others
-        gen_vs_sym(m)
+    only = {"vs_sym": gen_vs_sym, "vs_scale": gen_vs_scale}
+    if len(sys.argv) > 1 and sys.argv[1] in only:      # add this fixture without regenerating the others
+        only[sys.argv[1]](m)
         return
+    gen_vs_scale(m)
     gen_vs_sym(m)
     gen_vs_small(m)
     gen_vs_mid(m)

@@ -536,7 +536,7 @@ def test_voxel_selection_with_two_masks(dev, golden):
 
 def test_voxel_selection_ranking_vs_reference(dev, golden):
     """Full run on a planted-signal case: selected voxels and accuracies vs the reference's run."""
-    g = golden("vs_mid")
+    g = golden("vs_mid_run")
     raw = list(g["rawf"])
     labels = [int(x) for x in g["labelsf"]]
     clf = svm.SVC(kernel='precomputed', shrinking=False, C=1)
@@ -784,7 +784,7 @@ def test_gpu_shrink_matches_reference_rule(dev):
 
 def test_gpu_svm_cv_matches_sklearn(dev, golden):
     """Batched GPU SMO (libsvm restatement) vs sklearn.cross_val_score on the same kernels."""
-    g = golden("vs_mid")
+    g = golden("vs_mid_run")
     # (a) the kernels the unmodified reference built in its full run -> the accuracies it reported
     Kf = np.ascontiguousarray(g["kernelsf"])
     labels = [int(x) for x in g["labelsf"]]
@@ -887,7 +887,7 @@ def test_gpu_svm_cv_multiclass_matches_sklearn(dev):
 
 
 def test_voxel_selector_gpu_cv_equals_host_cv(dev, golden):
-    g = golden("vs_mid")
+    g = golden("vs_mid_run")
     raw = list(g["rawf"])
     labels = [int(x) for x in g["labelsf"]]
     clf = svm.SVC(kernel='precomputed', shrinking=False, C=1)
@@ -1008,26 +1008,12 @@ def test_voxel_selector_multi_gpu_nccl(dev):
 
 # ------------------------------------------------------------------------------- round 2: BASELINE config shapes,
 # noise floor, host entry point of the symmetric pipeline, range packing
-def _reference_or_skip():
-    from oracle import reference
-    if not reference.available():
-        pytest.skip("oracle/_ref (the unmodified reference, oracle/build_ref.sh) is not built")
-    return reference.load()
-
-
-def _reference_rows(m, raw, labels, eps, folds, s0, n0, mask_self=False, host_cv=True):
-    """Rows [s0, s0+n0) through the UNMODIFIED reference's stages (voxelselector.py:492-505): shrunk kernels and
-    cross-validation accuracies.  mask_self: zero the self column after its normaliser (SURVEY Appendix B.2)."""
-    vs = m.VoxelSelector(labels, eps, folds, raw, voxel_unit=n0, process_num=0)
-    clf = svm.SVC(kernel='precomputed', shrinking=False, C=1)
-    corr = vs._correlation_computation((s0, n0))
-    m.fcma_extension.normalization(corr, eps)
-    if mask_self:
-        for i in range(n0):
-            corr[i, :, s0 + i] = 0
-    K = vs._prepare_for_cross_validation(corr, clf)
-    acc = np.array([a for _, a in vs._do_cross_validation(clf, K, (s0, n0))]) if host_cv else None
-    return K, acc
+# The vs_scale fixture holds what the UNMODIFIED reference's stages (voxelselector.py:492-509) returned for these inputs
+# (tests/golden/make_golden.py gen_vs_scale): shrunk kernels and cross-validation accuracies of sampled rows.  The inputs
+# are too large to store; the tests regenerate them and check them against a stored probe of input values first.
+def _check_probe(raw, idx, val):
+    got = np.array([raw[e][t, v] for e, t, v in idx], np.float32)
+    assert np.allclose(got, val, rtol=1e-5, atol=1e-7), "synthetic inputs differ from those the fixture was made from"
 
 
 def _gpu_rows_acc(K_rows, labels, folds):
@@ -1037,21 +1023,22 @@ def _gpu_rows_acc(K_rows, labels, folds):
 
 
 @pytest.mark.timeout(600)
-def test_config1_shape_vs_reference(dev):
+def test_config1_shape_vs_reference(dev, golden):
     """BASELINE configs[1] at FULL size (V=30 000, T=200, E=16, eps=8, fp32-faithful, one GPU): the symmetric pipeline
     (E=16 instantiations of the row and column passes, 8 passes of 4096 rows, ragged tail 30 000 = 117*256 + 48) against
     the unmodified reference on three 32-row samples: first pass, a middle pass, the ragged tail."""
-    m = _reference_or_skip()
+    g = golden("vs_scale")
     V, T, E, eps, folds = 30000, 200, 16, 8, 2
     raw, labels = synthetic.make_epochs(V, T, E)
+    _check_probe(raw, g["c1_probe_idx"], g["c1_probe"])
     ep, T_e = engine.stack_epochs(raw, dev)
     op = engine.pack_epochs(ep, T_e, "fp32")
     K = torch.zeros((V, E, E), device=dev)
     work = engine.SymWorkspace(E, V, 4096, dev, transposed_copy=False)
     engine.voxel_kernels_sym(op, 0, V, eps, work=work, out=K)
     same, total = 0, 0
-    for s0 in (64, 15008, V - 32):
-        Kref, acc_ref = _reference_rows(m, raw, labels, eps, folds, s0, 32)
+    assert list(g["c1_rows"]) == [64, 15008, V - 32]
+    for s0, Kref, acc_ref in zip(g["c1_rows"], g["c1_kernels"], g["c1_acc"]):
         Kg, acc = _gpu_rows_acc(K[s0:s0 + 32], labels, folds)
         assert np.max(np.abs(Kg - Kref)) <= 3e-5 * np.max(np.abs(Kref))      # measured 1.3e-5 (reference's own ssyrk noise ~1e-5)
         same += int(np.sum(acc == acc_ref))
@@ -1061,14 +1048,15 @@ def test_config1_shape_vs_reference(dev):
 
 
 @pytest.mark.timeout(600)
-def test_config4_classifier_kernel_at_scale(dev):
+def test_config4_classifier_kernel_at_scale(dev, golden):
     """BASELINE configs[4] shape class (Classifier precomputed kernel, one mask, V = 20 000, E = 32): the one [E, E]
     kernel of engine.classifier_kernel equals the fp64 sum of the per-voxel kernels, and sampled per-voxel kernels equal
     the unmodified reference's (its own full classifier run at this size is ~10 min of CPU: classifier.py:279-348 is the
     same per-row arithmetic summed over rows, pinned at small size by test_classifier_big_kernel_vs_reference)."""
-    m = _reference_or_skip()
+    g = golden("vs_scale")
     V, T, E, eps = 20000, 200, 32, 8
     raw, labels = synthetic.make_epochs(V, T, E)
+    _check_probe(raw, g["c4_probe_idx"], g["c4_probe"])
     ep, T_e = engine.stack_epochs(raw, dev)
     op = engine.pack_epochs(ep, T_e, "fp32")
     Kc = engine.classifier_kernel(op, op, 0, V, eps)
@@ -1076,8 +1064,12 @@ def test_config4_classifier_kernel_at_scale(dev):
     Ksum = Kv.to(torch.float64).sum(0)
     assert float((Kc.to(torch.float64) - Ksum).abs().max()) <= 2e-6 * float(Ksum.abs().max())
     assert float((Kc - Kc.t()).abs().max()) == 0.0 or float((Kc - Kc.t()).abs().max()) <= 1e-6 * float(Kc.abs().max())
-    for s0 in (256, 10016, V - 32):
-        Kref, _ = _reference_rows(m, raw, labels, eps, 4, s0, 32, host_cv=False)
+    assert list(g["c4_rows"]) == [256, 10016, V - 32]
+    iu = np.triu_indices(E)
+    for s0, Kref_triu in zip(g["c4_rows"], g["c4_kernels_triu"]):
+        Kref = np.zeros((32, E, E), np.float32)
+        Kref[:, iu[0], iu[1]] = Kref_triu
+        Kref[:, iu[1], iu[0]] = Kref_triu      # the reference's kernels are symmetric (checked when the fixture is made)
         Kg, _ = _gpu_rows_acc(Kv[s0:s0 + 32], labels, 4)
         assert np.max(np.abs(Kg - Kref)) <= 3e-5 * np.max(np.abs(Kref))
     # the classifier's decimal shrink rule (classifier.py:343-347) on the summed kernel
@@ -1086,22 +1078,20 @@ def test_config4_classifier_kernel_at_scale(dev):
 
 
 @pytest.mark.timeout(900)
-def test_result_level_noise_floor(dev):
-    """SURVEY Appendix B.2 result-level contract, measured in this run: with the self column present ("drop-in" mode)
-    even the reference re-run on TR-permuted inputs (identical mathematics) changes the accuracy of a large share of the
-    chance-level voxels; a precision mode must not disagree with the reference more than that noise floor (plus a small
+def test_result_level_noise_floor(dev, golden):
+    """SURVEY Appendix B.2 result-level contract, against the reference's accuracies in vs_scale: with the self column
+    present ("drop-in" mode) even the reference re-run on TR-permuted inputs (identical mathematics) changes the accuracy
+    of a large share of the chance-level voxels; a precision mode must not disagree with the reference more than that noise floor (plus a small
     margin), and must agree almost everywhere once the self column is masked on both sides."""
-    m = _reference_or_skip()
+    g = golden("vs_scale")
     V, T, E, eps, folds = 768, 200, 32, 8, 4
     raw, labels = synthetic.make_epochs(V, T, E)
-    perm = np.random.RandomState(7).permutation(T)
-    raw_p = [np.ascontiguousarray(x[perm]) for x in raw]
-    _, acc_ref = _reference_rows(m, raw, labels, eps, folds, 0, V)
-    _, acc_perm = _reference_rows(m, raw_p, labels, eps, folds, 0, V)
-    floor = float(np.mean(acc_ref != acc_perm))            # e.g. 0.1 - 0.2 (SURVEY: 352 / 2000)
-    Kref_m, _ = _reference_rows(m, raw, labels, eps, folds, 0, V, mask_self=True, host_cv=False)
-    # masked reference accuracies through the batched GPU SVM (== scikit-learn, test_gpu_svm_cv_matches_sklearn)
-    acc_ref_m = engine.svm_cv_precomputed(torch.from_numpy(Kref_m).to(dev), labels, folds, C=1.0, tol=1e-3)
+    _check_probe(raw, g["nf_probe_idx"], g["nf_probe"])
+    # the reference's accuracies on these inputs and on the inputs with their TRs permuted (RandomState(7).permutation(T))
+    acc_ref, acc_perm = g["nf_acc"], g["nf_acc_perm"]
+    floor = float(np.mean(acc_ref != acc_perm))            # measured 0.33 (SURVEY: 352 / 2000)
+    # the reference's accuracies (its own scikit-learn cross-validation) with the self column masked
+    acc_ref_m = g["nf_acc_masked"]
     planted = set(range(V // 100))
     clf = svm.SVC(kernel='precomputed', shrinking=False, C=1)
     bounds = {"fp32": (1.25, 0.02, 0.99), "tf32x3": (1.25, 0.02, 0.99), "bf16x3": (1.25, 0.02, 0.985),

@@ -5,7 +5,7 @@ import os, sys, numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from sklearn import svm
 from brainiak_b200.fcma.voxelselector import VoxelSelector
-g = np.load(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "vs_mid.npz"))
+g = np.load(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "vs_mid_run.npz"))
 raw = list(g["rawf"]); labels = [int(x) for x in g["labelsf"]]; ref = g["accf"]
 clf = svm.SVC(kernel='precomputed', shrinking=False, C=1)
 for prec in ("fp32", "fp16x3", "tf32x3", "bf16x3", "tf32", "bf16"):
